@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the lens-warp benchmark (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 metric   lens-warp Mpixels/s (output pixels, W*H per frame) on the headline workload of
          BASELINE.json: 3840x2160 screen, cube globe of 6x2048^2 8-bit faces, panini lens.
@@ -25,6 +25,8 @@ secondary  every other BASELINE configuration (C2, C3, the C4 lenses, C5 trism/c
          cold frame, same three fractions.
 --impl reference   the reference's own CPU loop (oracle/_ref = unmodified fisheye.c compiled
          headless; else the oracle port) on the host cores, same workload, bounded sample.
+--dump-outputs DIR  after the timed steps, rank 0's output batch of the last step as a fixed, seeded sample
+         (see dump_outputs); the inputs are seeded too, so two builds can be compared output for output.
 
 The oracle (oracle/) is only ever the thing TIMED BESIDE or CHECKED AGAINST — never the
 product path, which raises if libblinky_b200.so is missing.
@@ -327,6 +329,23 @@ def roofline_entry(fe, launch_s, frames, peak, traffic):
     return out
 
 
+DUMP_SAMPLE = 1 << 22  # drawn pixel positions: <= 16 MB of float32 values + 32 MB of float64 indices
+
+
+def dump_outputs(directory, d_out):
+    """What a caller of the timed path receives, d_out [frames][H][W] uint8, sampled at a fixed seeded set of
+    positions (the whole batch is 531 MB as float32): out.npy holds the pixel values as float32, out_index.npy
+    their flat indices into d_out as float64, both in ascending index order."""
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    flat = d_out.reshape(-1)
+    idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), DUMP_SAMPLE))
+    vals = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    np.save(os.path.join(directory, "out.npy"), vals.astype(np.float32))
+    np.save(os.path.join(directory, "out_index.npy"), idx.astype(np.float64))
+
+
 def load_traffic():
     """measured DRAM bytes per launch (ncu, this round) per workload: profiles/traffic_r2.json, written by
     scripts/ncu_traffic.py from the committed .ncu-rep summaries"""
@@ -352,7 +371,12 @@ def main():
     ap.add_argument("--gather-mode", default="best", choices=["best", "nccl", "peer_copy", "peer_store"],
                     help="N > 1: which transport's delivered rate is `value` (best = the fastest of the three measured)")
     ap.add_argument("--chunk", type=int, default=4, help="frames per gather chunk (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's output to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's output; the reference arm keeps none")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -421,6 +445,8 @@ def main():
     launches = fe.launch_count - launches0
     elapsed = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
     kernel_name = fe.last_kernel
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out)
     # the timed region is a few milliseconds: keep the identical load running so that NVML
     # (which refreshes every few ms) actually sees the clocks this kernel runs at
     t_end = time.time() + 1.0

@@ -101,12 +101,33 @@ static void to_cmd(const char *command, void *user)
     Cmd_ExecuteString(command, src_command); /* a lens's `onload` may be any console command */
 }
 
+/* A context's first blinky_warp_host sets up its copy pipeline (streams, device slots, pinned
+ * staging): tens of milliseconds.  The back context pays that here, on the worker, with the kinds of
+ * buffers F_RenderView passes (pinned faces, an unpinned screen, keep_unmapped), instead of in the
+ * first frame after the swap.  Best effort: a failure here only moves the cost back to that frame. */
+static void warm_up(blinky_ctx *c)
+{
+    size_t faces = (size_t)build_ps * build_ps * BLINKY_MAX_PLATES;
+    void *src = NULL;
+    byte *dst;
+
+    if (blinky_alloc_pinned(c, faces, &src) != BLINKY_OK) return;
+    memset(src, 0, faces);
+    dst = malloc((size_t)build_w * build_h);
+    if (dst) {
+        blinky_warp_host(c, src, faces, dst, 0, build_w, 0, 0, 1, 1);
+        free(dst);
+    }
+    blinky_free_pinned(c, src);
+}
+
 static void *build_worker(void *arg)
 {
     (void)arg;
     /* errors (invalid lens, zoom failure, ...) are collected in the context's log and printed by the
      * main thread at the swap; like the reference, an empty map simply draws nothing */
     blinky_build_lensmap(ctx[1 - front], build_w, build_h, build_ps, build_threads);
+    warm_up(ctx[1 - front]);
     __sync_synchronize();
     build_done = 1;
     return NULL;

@@ -30,6 +30,25 @@ def _p(a):
     return a.ctypes.data_as(c_void_p)
 
 
+_short_dirs = {}
+
+
+def _short_basedir(basedir: str) -> str:
+    """The reference formats "<basedir>/lua-scripts/lenses/<name>.lua" into a char[100] with sprintf
+    (engine/NQ/fisheye.c:1665-1666, 1758-1759): from a checkout a few directories deep the longer lens
+    names overflow it and the process aborts.  It gets the directory through a short symlink instead."""
+    if basedir not in _short_dirs:
+        import atexit
+        import shutil
+        import tempfile
+
+        d = tempfile.mkdtemp(prefix="bref")
+        atexit.register(shutil.rmtree, d, True)
+        os.symlink(os.path.abspath(basedir), os.path.join(d, "s"))
+        _short_dirs[basedir] = os.path.join(d, "s")
+    return _short_dirs[basedir]
+
+
 # ---------------------------------------------------------------------------
 # the compiled reference
 # ---------------------------------------------------------------------------
@@ -60,13 +79,13 @@ class RefOracle:
         L.ref_lens_inverse.argtypes = [c_double, c_double, c_void_p]
         L.ref_lens_forward.argtypes = [c_void_p, POINTER(c_double), POINTER(c_double)]
         self.palette = np.ascontiguousarray(palette, np.uint8).reshape(768)
-        rc = L.ref_init(basedir.encode(), _p(self.palette))
+        rc = L.ref_init(_short_basedir(basedir).encode(), _p(self.palette))
         if rc != 0:
             raise RuntimeError("ref_init failed (already initialised in this process?)")
         self.W = self.H = 0
 
     def set_basedir(self, basedir: str):
-        self.lib.ref_set_basedir(basedir.encode())
+        self.lib.ref_set_basedir(_short_basedir(basedir).encode())
 
     def command(self, text: str):
         self.lib.ref_command(text.encode())

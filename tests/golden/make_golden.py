@@ -2,7 +2,7 @@
 i.e. the unmodified /root/reference/engine/NQ/fisheye.c) driving the repo's own
 script set.  Run here (needs oracle/_ref built):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 Outputs (all under tests/golden/):
   lensmaps_small.npz   idx/tint per (globe, lens) at 128x96, plates 48
@@ -14,12 +14,19 @@ Outputs (all under tests/golden/):
   engine_frame.npz     whole F_RenderView frames (platesize = min(w,h))
   palmaps.npz          the six rubix LUTs for the seeded palette
   config.txt           F_WriteConfig output
+  reference_live.json  the reference's side of every test that used to drive the compiled
+                       reference live (lensmap digests of every globe x lens, console
+                       and config text, rendered frame digests, the reference's own
+                       scripts run by the product)
+  reference_pcx.npz    f_saveglobe PCX files written by the reference
 
-The GPU box has no /root/reference: tests there compare against these files.
+The tests compare against these files only, so they need neither the reference
+checkout nor oracle/_ref.
 """
 import hashlib
 import json
 import os
+import shutil
 import sys
 
 import numpy as np
@@ -137,8 +144,158 @@ def main():
     txt = R.write_config("/tmp/_blinky_cfg.txt")
     open(os.path.join(OUT, "config.txt"), "w").write(txt)
     R.command("f_rubixgrid 10 4 1")
+    reference_live(R, pal, sys.argv[1])
     print("golden vectors written to", OUT)
 
 
+def lensmap_digest(R, w, h, ps):
+    rc = R.build(w, h, ps)
+    idx, tint = R.lensmap()
+    return dict(rc=rc, idx_sha=sha(idx), tint_sha=sha(tint), scale=R.scale, display=R.display(), plates_sha=sha(R.plates()),
+                log=R.log)
+
+
+def reference_live(R, pal, reference_dir):
+    """The reference's results for the command sequences of the tests that compare with it
+    (tests/test_host.py, test_oracle.py, test_gpu_parity.py, test_dropin.py)."""
+    import tempfile
+
+    tmp = tempfile.mkdtemp()
+    cfg = os.path.join(tmp, "config.cfg")
+    live = {}
+
+    # every globe x lens at two sizes (test_host: all combinations; test_oracle: the restatement)
+    for key, (w, h, ps) in (("combos_96x64x40", (96, 64, 40)), ("combos_200x150x100", (200, 150, 100))):
+        R.set_screen(w, h)
+        live[key] = {}
+        for g in GLOBES:
+            for l in LENSES:
+                R.clear_log()
+                R.command(f"f_globe {g}")
+                R.command(f"f_lens {l}")
+                live[key][f"{g}__{l}"] = lensmap_digest(R, w, h, ps)
+
+    # the reference's own lua-scripts, run by the product (test_host: own scripts equal the reference's)
+    scripts = {}
+    with bb.Fisheye(device=None, basedir=os.path.join(reference_dir, "game"), palette=pal) as fe:
+        for g in GLOBES:
+            for l in LENSES:
+                fe.clear_log()
+                fe.command(f"f_globe {g}")
+                fe.command(f"f_lens {l}")
+                try:
+                    fe.build_lensmap(112, 80, 56, 4)
+                    rc = 0
+                except bb.BlinkyError as e:
+                    rc = e.code
+                idx, tint = fe.lensmap()
+                scripts[f"{g}__{l}"] = dict(rc=rc, idx_sha=sha(idx), tint_sha=sha(tint), scale=fe.scale, display=fe.display(),
+                                            log=fe.log, onload=fe.onload, max_fov=fe.max_fov, max_vfov=fe.max_vfov,
+                                            lens_width=fe.lens_width, lens_height=fe.lens_height, map_type=fe.map_type)
+    live["reference_scripts_112x80x56"] = scripts
+
+    # console surface (test_host)
+    for c in ("fisheye 1", "f_globe cube", "f_lens panini", "f_fov 180", "f_rubixgrid 10 4 1"):
+        R.command(c)
+    if R.rubix_enabled:
+        R.command("f_rubix")
+    R.clear_log()
+    for c in CONSOLE_SCRIPT:
+        R.command(c)
+    # the ERROR: lines are luaL_loadfile's message, which names the reference's script directory; the test
+    # ignores them (the product words its file-open errors differently)
+    log = "\n".join(x for x in R.log.split("\n") if not x.startswith("ERROR:"))
+    live["console"] = dict(log=log, config=R.write_config(cfg))
+
+    # f_saveglobe PCX files (test_host)
+    pcx, saveglobe_logs = {}, {}
+    w, h = 48, 40
+    ps = min(w, h)
+    R.set_screen(w, h)
+    with tempfile.TemporaryDirectory() as d:
+        R.lib.ref_set_write_dir(d.encode())
+        for globe in ("cube", "trism", "fast"):
+            for margins in (0, 1):
+                R.command(f"f_globe {globe}")
+                R.command("f_lens equirect")
+                faces = bb.synthetic_faces(R.numplates, ps, 6)
+                R.command(f"f_saveglobe g{margins}_ {margins}")
+                R.clear_log()
+                R.frame(faces, bb.synthetic_background(w, h))
+                saveglobe_logs[f"{globe}__{margins}"] = R.log
+                for i in range(R.numplates):
+                    pcx[f"{globe}__g{margins}_{i}"] = np.frombuffer(open(os.path.join(d, f"g{margins}_{i}.pcx"), "rb").read(), np.uint8)
+    live["saveglobe_logs"] = saveglobe_logs
+    np.savez_compressed(os.path.join(OUT, "reference_pcx.npz"), **pcx)
+
+    # rendered frames at 320x200 (test_gpu_parity)
+    frames = {}
+    W, H, PS = 320, 200, 128
+    R.set_screen(W, H)
+    for g, l, rubix in LIVE_FRAMES:
+        R.command(f"f_globe {g}")
+        R.command(f"f_lens {l}")
+        if R.rubix_enabled != rubix:
+            R.command("f_rubix")
+        R.build(W, H, PS)
+        frames[f"{g}__{l}__rubix{int(rubix)}"] = sha(R.render(bb.synthetic_faces(R.numplates, PS, 9), bb.synthetic_background(W, H)))
+    if R.rubix_enabled:
+        R.command("f_rubix")
+    live["frames_320x200x128"] = frames
+
+    # the drop-in's engine seam: console, whole F_RenderView frames, config (test_dropin)
+    for c in ("fisheye 1", "f_globe cube", "f_lens panini", "f_fov 180", "f_rubixgrid 10 4 1"):
+        R.command(c)
+    if R.rubix_enabled:
+        R.command("f_rubix")
+    R.clear_log()
+    for c in DROPIN_CONSOLE:
+        R.command(c)
+    dropin = {"log": R.log, "frames": {}}
+    for g, l, rubix, scr in DROPIN_FRAMES:
+        R.command(f"f_globe {g}")
+        R.command(f"f_lens {l}")
+        if R.rubix_enabled != rubix:
+            R.command("f_rubix")
+        w, h, rowbytes, vx, vy, vw, vh = scr
+        R.set_screen(w, h, rowbytes, vx, vy, vw, vh)
+        faces = bb.synthetic_faces(R.numplates, min(vw, vh), 4)
+        out, ncalls = R.frame(faces, np.random.default_rng(3).integers(0, 256, (h, w), dtype=np.uint8))
+        dropin["frames"][f"{g}__{l}"] = dict(sha=sha(out), calls=ncalls)
+    if R.rubix_enabled:
+        R.command("f_rubix")
+    dropin["config"] = R.write_config(cfg)
+    # 640x480 frames before and after an f_lens change (test_dropin: the rebuild never holds a frame up)
+    for c in ("fisheye 1", "f_globe cube", "f_lens panini", "f_fov 180"):
+        R.command(c)
+    if R.rubix_enabled:
+        R.command("f_rubix")
+    R.set_screen(640, 480, 640, 0, 0, 640, 480)
+    faces = bb.synthetic_faces(6, 480, 9)
+    bg = np.random.default_rng(5).integers(0, 256, (480, 640), dtype=np.uint8)
+    dropin["rebuild_old_sha"] = sha(R.frame(faces, bg)[0])
+    R.command("f_lens winkeltripel")
+    R.command("f_contain")
+    dropin["rebuild_new_sha"] = sha(R.frame(faces, bg)[0])
+    live["dropin"] = dropin
+
+    json.dump(live, open(os.path.join(OUT, "reference_live.json"), "w"), indent=0, sort_keys=True)
+    shutil.rmtree(tmp)
+
+
+CONSOLE_SCRIPT = ["fisheye 1", "f_rubixgrid 10 4 1", "fisheye", "fisheye 0", "fisheye 1", "f_help", "f_rubix", "f_rubix", "f_rubixgrid",
+                  "f_rubixgrid 7 3.5 0.25", "f_rubixgrid", "f_fov", "f_fov 100", "f_fov", "f_vfov 60", "f_vfov", "f_cover", "f_fov",
+                  "f_contain", "f_fov", "f_lens", "f_globe", "f_lens hammer", "f_lens", "f_globe trism", "f_globe", "f_lens nosuchlens",
+                  "f_globe nosuchglobe", "f_lens panini", "f_globe cube", "f_rubixgrid 10 4 1", "F_FOV 90"]
+LIVE_FRAMES = [("cube", "panini", True), ("trism", "stereographic", False), ("tetra", "hammer", True), ("cube", "winkeltripel", True),
+               ("fast", "panini", False), ("cube", "polyconic", True)]
+DROPIN_CONSOLE = ["f_help", "f_fov", "f_lens hammer", "f_lens", "f_globe trism", "f_globe", "f_rubix", "f_rubix", "f_vfov 70", "f_cover",
+                  "f_rubixgrid", "fisheye", "f_lens panini", "f_globe cube"]
+DROPIN_FRAMES = [("cube", "panini", False, (96, 64, 96, 0, 0, 96, 64)), ("cube", "fisheye1", True, (128, 80, 136, 16, 8, 96, 64)),
+                 ("trism", "equirect", True, (96, 64, 96, 0, 0, 96, 64)), ("tetra", "winkel1", False, (104, 72, 104, 8, 8, 88, 56))]
+
+
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_golden.py <reference checkout (its game/ holds the reference's lua-scripts)>")
     main()

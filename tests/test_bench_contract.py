@@ -29,6 +29,31 @@ def test_reference_arm_prints_one_json_line(bb):
     assert d["config"]["workload"] == "c1-640x480"
 
 
+@pytest.mark.gpu
+def test_dump_outputs_are_reproducible_and_steps_are_honoured(bb, cuda_device, tmp_path):
+    """--dump-outputs: the sampled output of the last timed step is float data under 64 MB and the same from run
+    to run (seeded inputs); --steps sets how many launches are timed"""
+    import numpy as np
+
+    dumps, per_step = [], set()
+    for steps in (2, 5):
+        d = tmp_path / f"steps{steps}"
+        r = run_bench("--workload", "c1-640x480", "--steps", str(steps), "--warmup", "1", "--no-secondary", "--no-cpu-baseline",
+                      "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.strip()][-1])
+        assert line["steps"] == steps and line["gpu_launches"] % steps == 0
+        per_step.add(line["gpu_launches"] // steps)
+        files = sorted(os.listdir(d))
+        assert files == ["out.npy", "out_index.npy"]
+        assert sum(os.path.getsize(d / f) for f in files) <= 64 << 20
+        dumps.append({f: np.load(d / f) for f in files})
+    assert len(per_step) == 1 and per_step.pop() >= 1
+    for f in dumps[0]:
+        assert dumps[0][f].dtype in (np.float32, np.float64) and dumps[0][f].size > 0
+        assert np.array_equal(dumps[0][f], dumps[1][f]), f
+
+
 def test_product_arm_needs_a_gpu():
     import torch
 
